@@ -1,6 +1,7 @@
 """Benchmark of the CFR hot path (BASELINE.json metric: CFR+ iterations/s, beside the CPU path on the same box).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload fhp|leduc_b5|leduc_b3|leduc_pot]
+                    [--dump-outputs DIR]
 
 A "step" = one full CFR+ iteration (both seats: value/regret sweep + reach/average sweep each) over the whole public
 tree, with the exact best-response evaluation of the current AND the average strategy every `--eval-every` iterations
@@ -479,6 +480,8 @@ def main_fhp(a, rank, world, local_rank):
         dist.barrier()
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     max_ms = float(t.item())
+    if a.dump_outputs and rank == 0:  # before the roofline launches below change the tables
+        dump_outputs(a.dump_outputs, board_engine_outputs(s, trace))
 
     # --- roofline of the dominant kernel (board_sweep_kernel, update form), CUDA events on its stream around each launch
     def ev_pair():
@@ -651,6 +654,41 @@ def s_n_boards(n, rank, world):
     return len(range(rank, n, world))
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_BOARDS = 256  # 256 boards x 2 tables x 14 rows x 1088 floats = 30.5 MB
+
+
+def board_engine_outputs(s, trace):
+    """What a caller of the timed fhp path receives - BoardCFRSolver.state_dict() and the exploitability trace - with the
+    per-board tables cut to the rows of a fixed, seeded sample of DUMP_BOARDS of this rank's boards, each board's rows in the
+    order of the post-deal tree's nodes: [boards, rows per board, ldb]."""
+    import numpy as np
+    import torch
+    s.flush_average()
+    rng = np.random.default_rng(0)
+    boards = np.sort(rng.choice(s.n_boards, min(DUMP_BOARDS, s.n_boards), replace=False))
+    own_rows = [r0 for _, (r0, _) in sorted(s.local_rows.items())]
+    rows = torch.from_numpy((boards[:, None] * s.rows_per_board + np.array(own_rows)[None, :]).reshape(-1)).to(s.regret.device)
+    shape = (boards.size, len(own_rows), s.regret.shape[1])
+    return {"exploitability": np.array(trace, np.float64).reshape(-1, 3),  # (iteration, current, average) in mbb/g
+            "regret_rows": s.regret[rows].cpu().numpy().reshape(shape), "avg_rows": s.avg[rows].cpu().numpy().reshape(shape),
+            "trunk_regret": s.bufs.regret.cpu().numpy(), "trunk_strat": s.bufs.strat.cpu().numpy(),
+            "trunk_avg": s.bufs.avg.cpu().numpy()}
+
+
+def dump_outputs(out_dir, arrays):
+    """out_dir/<name>.npy for every array (float32 / float64 only, at most DUMP_LIMIT_BYTES in all)"""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("outputs of %d bytes exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError("%s: dtype %s is neither float32 nor float64" % (name, a.dtype))
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -683,7 +721,14 @@ def main():
     ap.add_argument("--converge", type=int, default=0, metavar="ITERS",
                     help="fhp / hulh: run ITERS iterations and print the exploitability-vs-wall-clock curve (one JSON line) "
                          "instead of the throughput line; evaluation every --eval-every iterations")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="fhp: after the timed steps write what they computed as DIR/<name>.npy (float32 / float64, <= 64 MB: "
+                         "exploitability trace, trunk tables, the table rows of a fixed seeded sample of %d boards)" % DUMP_BOARDS)
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.workload != "fhp" or a.impl != "b200" or a.converge):
+        ap.error("--dump-outputs covers the timed GPU run of the fhp workload")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,7 +1,7 @@
 """Probe: full Flop5Holdem (134 459 isomorphism classes) on one GPU - build time, memory, iteration time."""
-import sys, time
+import os, sys, time
 import torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from pokerrl_b200.game import games
 from pokerrl_b200.game.flat_tree import FlatTree
 from pokerrl_b200.game.holdem_boards import BoardSpec

@@ -1,5 +1,5 @@
-import sys, ctypes as C, torch, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, ctypes as C, torch, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from bench import make_tree
 from pokerrl_b200 import _native as nat
 from pokerrl_b200.solver import CFRSolver
