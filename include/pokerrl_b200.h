@@ -430,6 +430,54 @@ int prl_env_step(const prl_env_cfg_t* cfg, int32_t* state, int8_t* deck, const i
                  double* rewards, uint8_t* done, uint8_t* legal, uint64_t seed, uint64_t step_id, int auto_reset,
                  prl_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * Head-to-head play of two tabular agents (replaces the per-hand loop of
+ * PokerRL/eval/head_to_head/LocalHead2HeadMaster.py:81-126).  One table of the batched env per hand; each table walks
+ * the agents' shared public tree in step with its env.  Hands [0, n_hands_per_seat) have agent A in seat 0, the rest
+ * agent A in seat 1.  Host loop: prl_h2h_step, then prl_env_step with the actions it wrote, at most "tree depth" times,
+ * one more prl_h2h_step, then prl_h2h_collect.
+ * ------------------------------------------------------------------------------------------------------------------ */
+typedef struct {
+    int32_t n_envs;           /* tables in this batch (= prl_env_cfg_t.n_envs) */
+    int32_t n_range;          /* hands per seat (RANGE_SIZE) */
+    int32_t n_hole;           /* 1: hand = card, chance child = rank of the dealt card among the cards not on the board;
+                                 2: hand = lexicographic index of (c1 < c2) */
+    int32_t chance_by_class;  /* 1: chance child = board_class[lexicographic rank of the sorted 5-card board] */
+    int32_t max_decisions;    /* row width of `uniforms` */
+    int64_t seat_swap_at;     /* global hands >= this one have agent A in seat 1 */
+    int64_t hand0;            /* global index of this batch's first hand (counter RNG, seat assignment) */
+    uint64_t seed;
+    const int8_t* kind;       /* DEVICE int8[n_nodes]  flat tree (game/flat_tree.py) */
+    const int32_t* first_child, *n_children, *first_slot, *action;
+    const float* table_a;     /* DEVICE float32[n_slots][ld_a]: agent A's action probabilities */
+    const float* table_b;
+    int64_t ld_a, ld_b;
+    const int32_t* board_class; /* DEVICE int32[C(52,5)] or NULL */
+    const uint8_t* board_perm;  /* DEVICE uint8[C(52,5)]: suit permutation s mapping the board onto its class */
+    const int16_t* sym_perm;    /* DEVICE int16[24][n_range]: hand h on the board reads row sym_perm[s][h] */
+    const double* uniforms;     /* DEVICE float64[n_envs][max_decisions] (replays) or NULL: counter RNG (seed, hand, k) */
+    int32_t* node;            /* DEVICE int32[n_envs]  per-table tree node, -1 after a desync */
+    int32_t* n_dec;           /* DEVICE int32[n_envs]  decisions taken so far */
+    uint8_t* perm;            /* DEVICE uint8[n_envs]  suit permutation of the dealt board */
+    int32_t* chips;           /* DEVICE int32[n_envs]  agent A's chip result once the hand ended */
+    unsigned long long* desync; /* DEVICE uint64[1]    invariant violations (acting seat / terminal state) */
+} prl_h2h_t;
+
+/* Starts every table at the root (node 0, no decision taken). */
+int prl_h2h_init(const prl_h2h_t* h, int32_t* actions, prl_stream_t stream);
+
+/* Moves each table's node by actions[i] (the action the env just applied) and through a chance node by the dealt board,
+ * checks the node against the env (state / deck / rewards of prl_env_step), and writes the next action of a table whose
+ * node is a decision node, sampled like EvalAgentBase.get_action; -1 where the hand is over. */
+int prl_h2h_step(const prl_h2h_t* h, const prl_env_cfg_t* cfg, const int32_t* state, const int8_t* deck,
+                 const double* rewards, int32_t* actions, prl_stream_t stream);
+
+/* Tables whose node is not terminal here (a hand the loop did not finish) count as desyncs.
+ * sums[0] += sum of agent A's chip results, sums[1] += sum of their squares (DEVICE int64[2]); winnings = DEVICE
+ * float32[n_envs] or NULL: chips / REWARD_SCALAR * REWARD_SCALAR * ev_normalizer per hand. */
+int prl_h2h_collect(const prl_h2h_t* h, double reward_scalar, double ev_normalizer, long long* sums, float* winnings,
+                    prl_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -74,6 +74,16 @@ class PrlEnvCfg(C.Structure):
     ]
 
 
+class PrlH2H(C.Structure):
+    _fields_ = [("n_envs", C.c_int32), ("n_range", C.c_int32), ("n_hole", C.c_int32), ("chance_by_class", C.c_int32),
+                ("max_decisions", C.c_int32), ("seat_swap_at", C.c_int64), ("hand0", C.c_int64), ("seed", C.c_uint64),
+                ("kind", C.c_void_p), ("first_child", C.c_void_p), ("n_children", C.c_void_p), ("first_slot", C.c_void_p),
+                ("action", C.c_void_p), ("table_a", C.c_void_p), ("table_b", C.c_void_p), ("ld_a", C.c_int64),
+                ("ld_b", C.c_int64), ("board_class", C.c_void_p), ("board_perm", C.c_void_p), ("sym_perm", C.c_void_p),
+                ("uniforms", C.c_void_p), ("node", C.c_void_p), ("n_dec", C.c_void_p), ("perm", C.c_void_p),
+                ("chips", C.c_void_p), ("desync", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -159,6 +169,11 @@ def lib():
     L.prl_env_step.argtypes = [ep, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                C.c_uint64, C.c_uint64, C.c_int, C.c_void_p]
     L.prl_env_reset.restype = L.prl_env_step.restype = C.c_int
+    hp = C.POINTER(PrlH2H)
+    L.prl_h2h_init.argtypes = [hp, C.c_void_p, C.c_void_p]
+    L.prl_h2h_step.argtypes = [hp, ep, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.prl_h2h_collect.argtypes = [hp, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.prl_h2h_init.restype = L.prl_h2h_step.restype = L.prl_h2h_collect.restype = C.c_int
     _lib = L
     return L
 

@@ -26,6 +26,7 @@ SOURCES = {
     "env_kernels.cu": [],
     "lbr_rollout.cu": [],
     "allin_dense.cu": [],
+    "h2h.cu": [],
 }
 
 

@@ -15,16 +15,14 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "env_state.cuh"
 #include "hand_eval.cuh"
 #include "pokerrl_b200.h"
 #include "prl_common.cuh"
 
 namespace {
 
-enum Field {
-    F_ROUND, F_POT, F_STACK0, F_STACK1, F_BET0, F_BET1, F_FLAGS, F_CUR, F_LAST_RAISER, F_N_ACT_EP, F_N_RAISES,
-    F_CAPPED, F_CAP_RAISER, F_CAP_NOREOPEN, F_LAST_TYPE, F_LAST_AMT, F_LAST_WHO, F_DONE, kFields
-};
+using namespace prl_env;
 enum { FL_ALLIN0 = 1, FL_ALLIN1 = 2, FL_FOLD0 = 4, FL_FOLD1 = 8, FL_ACTED0 = 16, FL_ACTED1 = 32 };
 enum { FOLD = 0, CALL = 1, RAISE = 2 };
 

@@ -176,3 +176,34 @@ class MultiStreetBoards:
             mult.append(np.ones(len(rows)))
         return MultiStreetBoards(boards, parents, prob, mult,
                                  "sub-game at board %s, %s boards per layer" % (list(root_board), [b.shape[0] for b in boards]))
+
+
+def board_class_map(spec):
+    """Deal map of a full-game, suit-isomorphic `BoardSpec` of a 52-card, 5-board-card game: for each of the C(52,5) boards,
+    indexed by the lexicographic rank of the sorted board (the order of `_combos_52_5`), the class it belongs to (int32, row
+    of `spec.boards`) and the suit permutation s (uint8, row of `spec.sym_perm`) that maps the board onto that class's
+    representative.  A hand h dealt on the board plays as hand `spec.sym_perm[s][h]` on the representative."""
+    reps, sp = np.asarray(spec.boards), spec.sym_perm
+    if sp is None or reps.shape != (134459, 5):
+        raise ValueError("a board -> class map needs the full game's suit-isomorphism classes (BoardSpec.full_game); a spec over "
+                         "a deck subset or without isomorphism has no strategy for most dealt boards")
+    if getattr(spec, "_class_map", None) is None:
+        boards = _combos_52_5().astype(np.int64)
+        rank, suit = boards // 4, boards % 4
+        rkey = np.zeros(reps.shape[0], np.int64)
+        for i in range(5):
+            rkey = rkey * 64 + reps[:, i].astype(np.int64)
+        cls = np.full(boards.shape[0], -1, np.int32)
+        perm = np.zeros(boards.shape[0], np.uint8)
+        for s, p in enumerate(permutations(range(4))):  # the row order of suit_permutation_hand_tables
+            m = np.sort(rank * 4 + np.array(p)[suit], axis=1)
+            k = np.zeros(m.shape[0], np.int64)
+            for i in range(5):
+                k = k * 64 + m[:, i]
+            pos = np.minimum(np.searchsorted(rkey, k), rkey.size - 1)
+            hit = (rkey[pos] == k) & (cls < 0)
+            cls[hit] = pos[hit]
+            perm[hit] = s
+        assert (cls >= 0).all()
+        spec._class_map = (cls, perm)
+    return spec._class_map
